@@ -2,6 +2,7 @@
 """Benchmark of the geometric propagate hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+                    [--dump-outputs DIR]
 
 Workload (N=1, and per rank for N>1 -- weak scaling): BASELINE.json configs[1],
 "Double-Gauss 12-surface, 1e7 rays, 3 wavelengths, FP64, 1xB200": one STEP is
@@ -184,6 +185,40 @@ def run_reference(args):
                 "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }))
+
+
+DUMP_RAYS = 12288          # rays per wavelength written by --dump-outputs
+
+
+def dump_outputs(path, eng, dev, N):
+    """--dump-outputs: the result arrays y, u, i, t of every wavelength bundle
+    as the timed step left them, for rays 0, step, 2*step, ... (DUMP_RAYS of
+    them, one strided D2H per surface row), float64, as <path>/<k>_l<li>.npy
+    with the ray indices in <path>/ray_index.npy.  A ray clipped by an
+    aperture or missing a surface is NaN in the trace from there on; every
+    file is kept finite, so non-finite entries are written as 0 and
+    <path>/<k>_l<li>_nonfinite.npy (float32, same shape) says what they were:
+    1 for NaN, +2 / -2 for +inf / -inf, 0 for a finite value.  The launch rays depend only on the seed, so two builds
+    given the same arguments can be compared array by array.
+    3 bundles x 12 surfaces x 10 values x (8 + 4) B x 12288 rays = 53 MB."""
+    from rayopt_b200._lib import check, ptr
+    count = min(N, DUMP_RAYS)
+    step = N//count
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "ray_index.npy"), np.arange(count, dtype=np.float64)*step)
+    for li, d in enumerate(dev):
+        for k in "YUIT":
+            a = d[k]
+            width = a.dtype.itemsize*(a.shape[2] if len(a.shape) == 3 else 1)
+            out = np.empty((a.shape[0], count) + tuple(a.shape[2:]), a.dtype)
+            for s in range(a.shape[0]):
+                check(eng.lib.rtx_memcpy2d_d2h(eng.ctx, ptr(out[s]), width, a.rows(s).ptr,
+                                               step*width, width, count))
+            eng.sync()
+            code = np.where(np.isnan(out), 1., np.where(np.isinf(out), 2.*np.sign(out), 0.))
+            name = os.path.join(path, "%s_l%d" % (k.lower(), li))
+            np.save(name + ".npy", np.where(np.isfinite(out), out, 0.))
+            np.save(name + "_nonfinite.npy", code.astype(np.float32))
 
 
 def rel_err(a, b):
@@ -479,7 +514,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-headline", action="store_true")
     ap.add_argument("--no-multi", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed step's results as .npy files")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -572,6 +611,10 @@ def main():
         step()
     barrier()
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs and rank == 0:
+        # the launches after the timed region repeat its step on the same
+        # inputs, so the arrays hold what the last timed step wrote
+        dump_outputs(args.dump_outputs, eng, dev, N)
     ms = maxr(ms)
     ms_per_step = ms/args.steps
     value = world*nl*N*S/(ms_per_step*1e-3)

@@ -132,36 +132,33 @@ def test_bound_reference_class_matches_reference():
             assert np.array_equal(np.asarray(xa), np.asarray(xb), equal_nan=True)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 def test_element_level_entry_points_match_reference():
     """rayopt_b200.elements.propagate / intercept / refract vs the reference's
     Spheroid methods (test_elements.py:109-134 style: a refracting sphere and
-    an asphere hit by random near-axis rays)."""
-    warnings.simplefilter("ignore")
-    R = ref_shim.load()
+    an asphere hit by random near-axis rays); the surfaces and the reference's
+    results are stored in tests/golden/pins/elements.json/.npz."""
+    import pins
     from rayopt_b200 import elements as el
+    meta, want = pins.load("elements")
     rng = np.random.default_rng(5)
     n = 100
     y0 = np.c_[rng.normal(0, .5, (n, 2)), -np.ones(n)]
     u0 = rng.normal(0, .02, (n, 2))
     u0 = np.c_[u0, np.sqrt(1 - np.square(u0).sum(1))]
     eng = OracleEngine()
-    for kw in (dict(curvature=.1, material=1.5), dict(curvature=-.05, conic=-.7, material="mirror"),
-               dict(curvature=.08, aspherics=[0, 1e-4, -2e-6], material=1.7), dict(material=1.3)):
-        kw = dict(kw)
-        kw["material"] = R.Material.make(kw["material"])
-        s = R.Spheroid(radius=1.2, **kw)
-        want = s.propagate(y0, u0, 1.1, 550e-9, clip=True)
-        got = el.propagate(s, y0, u0, 1.1, 550e-9, clip=True, engine=eng)
+    for j, rec in enumerate(meta["surfaces"]):
+        l = 550e-9
+        s = pins.PinnedElement(rec["attrs"], {repr(l): rec["n_mu"]})
+        got = el.propagate(s, y0, u0, 1.1, l, clip=True, engine=eng)
         tol = dict(rtol=1e-13, atol=1e-14)
-        np.testing.assert_allclose(got[0], want[0], **tol)
-        np.testing.assert_allclose(got[1], want[1], **tol)
-        assert got[2] == want[2]
-        np.testing.assert_allclose(got[3], want[3], **tol)
-        np.testing.assert_allclose(el.intercept(s, y0, u0, engine=eng), s.intercept(y0, u0), **tol)
-        mu = 1.1/want[2] if not s.material.mirror else -1.
-        ys = want[0]
-        np.testing.assert_allclose(el.refract(s, ys, u0, mu, engine=eng), s.refract(ys, u0, mu),
+        np.testing.assert_allclose(got[0], want["%d_y" % j], **tol)
+        np.testing.assert_allclose(got[1], want["%d_u" % j], **tol)
+        assert got[2] == rec["n"]
+        np.testing.assert_allclose(got[3], want["%d_t" % j], **tol)
+        np.testing.assert_allclose(el.intercept(s, y0, u0, engine=eng), want["%d_intercept" % j], **tol)
+        mu = 1.1/rec["n"] if not rec["mirror"] else -1.
+        ys = want["%d_y" % j]
+        np.testing.assert_allclose(el.refract(s, ys, u0, mu, engine=eng), want["%d_refract" % j],
                                    rtol=1e-12, atol=1e-13)
 
 

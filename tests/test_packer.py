@@ -55,19 +55,13 @@ def test_aim_matches_reference_golden():
 
 def test_aim_finite_restatement_vs_reference():
     """rays.aim_finite == FiniteConjugate.aim (rayopt/conjugates.py:137-166)
-    bit for bit (live reference only)"""
-    import pytest
-    import ref_shim
-    if not ref_shim.available():
-        pytest.skip("reference tree not present")
-    import warnings
-    warnings.simplefilter("ignore")
-    R = ref_shim.load()
+    bit for bit (the reference's results: tests/golden/pins/aim_finite.json)"""
+    import pins
     from rayopt_b200.rays import aim_finite
-    fc = R.conjugates.FiniteConjugate(radius=5., pupil=dict(type="radius", radius=3., distance=50.))
+    want, _ = pins.load("aim_finite")
     a = np.array(((-3., -2.5), (3., 2.5)))
     for z in (50., -40.):
         for yo in ((0, .7), (0., 0.), (.3, -.4)):
-            y, u = fc.aim(np.array(yo), disc(500, 2), z=z, a=a.copy(), surface=None, filter=False)
             hy, hu = aim_finite(yo, disc(500, 2), z, a, 5.)
-            assert np.array_equal(y, hy) and np.array_equal(u, hu)
+            w = want["%g_%g_%g" % ((z,) + yo)]
+            assert pins.digest(hy) == w["y"] and pins.digest(hu) == w["u"]
