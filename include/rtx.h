@@ -478,6 +478,41 @@ int rtx_focus_moments(rtx_ctx *ctx, int dtype, int64_t N, const void *y,
                       const void *inc, const void *w, const double *center,
                       double *m);
 
+/* ---- wavefront: OPD map and PSF (rayopt/geometric_trace.py:101-169) ------ */
+/*
+ * GeometricTrace.opd(resample) of a HEXAPOLAR launch bundle generated without
+ * a pupil filter (pupil_distribution("hexapolar"), rayopt/utils.py:180-186:
+ * N = 1 + 3*rings*(rings+1) rays, ring r of 6r rays starting at 1 + 3r(r-1)),
+ * regridded on the device.  From the DEVICE arrays A (N,), P (N,3) of
+ * rtx_trace_opd and the reference ray's A[ref] = a_ref and P[ref] = p_ref
+ * (host, 3 doubles): per ray t = -(A - a_ref)/lscale (lscale = l/scale) and
+ * (x, y) = P - p_ref; h = max |x|, |y| over rays whose x, y, t are finite
+ * (:135-139).  DEVICE map (n,n) receives t linearly interpolated at the
+ * nodes (x_i, y_j) = np.mgrid[-1:1:1j*n, -1:1:1j*n]*h, row i = x.  The
+ * triangulation is the structured one of the launch grid (6*rings^2
+ * triangles), not Delaunay: a triangle with a non-finite vertex is dropped,
+ * so vignetted gaps stay NaN, and nodes outside every triangle are NaN.  A
+ * node on a shared edge takes the value of the lowest-index triangle, so the
+ * map is bit-identical run to run.  Host outputs: *h (may be NULL) and
+ * *n_finite (may be NULL), the count of rays with finite x, y, t (0: no ray
+ * made it through).  Synchronises.
+ */
+int rtx_opd_regrid(rtx_ctx *ctx, int64_t N, const double *A, const double *P,
+                   double a_ref, const double *p_ref, double lscale, int rings,
+                   int64_t n, double *map, double *h, int64_t *n_finite);
+
+/*
+ * GeometricTrace.psf (rayopt/geometric_trace.py:150-157) of an n x n OPD map
+ * in waves (DEVICE, FP64, NaN outside the pupil): pupil function
+ * where(finite, exp(-2 pi i o), 0)/sqrt(count), its zero-padded 2-D DFT of
+ * size M x M, M = pad*n, and psf = |DFT|^2/M^2 into DEVICE psf (M,M) FP64.
+ * Any M: every 1-D DFT is a Bluestein convolution computed with the library's
+ * own power-of-two FFT; the first pass transforms only the n non-zero rows.
+ * Scratch of about 32*n*M bytes plus up to 1 GB for large M is taken from the
+ * stream-ordered allocator.  Asynchronous on the context stream.
+ */
+int rtx_psf(rtx_ctx *ctx, int64_t n, const double *map, int pad, double *psf);
+
 #ifdef __cplusplus
 }
 #endif

@@ -68,6 +68,9 @@ SYMBOLS = {
     "rtx_ipc_close": (_i, [_vp, _vp]),
     "rtx_trace_gather": (_i, [_vp, _vp, _i, _vp, _i, _i64, _vp, _vp, _i, _i, _vp, _vp, _i64,
                               _u]),
+    "rtx_opd_regrid": (_i, [_vp, _i64, _vp, _vp, C.c_double, _vp, C.c_double, _i, _i64, _vp,
+                            _vp, _vp]),
+    "rtx_psf": (_i, [_vp, _i64, _vp, _i, _vp]),
 }
 
 _lib = None

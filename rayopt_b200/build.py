@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "librtx.so")
 SOURCES = ["rtx.cu"]
-HEADERS = ["rtx_device.cuh", os.path.join("..", "..", "include", "rtx.h")]
+HEADERS = ["rtx_device.cuh", "rtx_psf.cuh", os.path.join("..", "..", "include", "rtx.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -4,6 +4,7 @@
 //        -Xcompiler -fPIC -o librtx.so rtx.cu
 #include "../../include/rtx.h"
 #include "rtx_device.cuh"
+#include "rtx_psf.cuh"
 
 #include <sched.h>
 #include <sys/syscall.h>
@@ -1703,6 +1704,196 @@ int rtx_focus_moments(rtx_ctx* ctx, int dtype, int64_t N, const void* y, const v
     }
     CK(cudaMemcpyAsync(m, ctx->d_moments, 8 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+}  // extern "C"
+
+// ---- wavefront: OPD regridding and PSF (rtx_psf.cuh) ------------------------
+namespace {
+
+// stream-ordered scratch, released on every return path
+struct Scratch {
+    cudaStream_t stream;
+    std::vector<void*> ptrs;
+    explicit Scratch(cudaStream_t s) : stream(s) {}
+    ~Scratch() {
+        for (void* p : ptrs) cudaFreeAsync(p, stream);
+    }
+    template <typename T>
+    int get(T** p, size_t count) {
+        *p = nullptr;
+        cudaError_t e = cudaMallocAsync((void**)p, count * sizeof(T), stream);
+        if (e != cudaSuccess) return (int)e;
+        ptrs.push_back(*p);
+        return 0;
+    }
+};
+
+int grid_for(rtx_ctx* ctx, long long work, int threads) {
+    long long b = (work + threads - 1) / threads, cap = (long long)ctx->sm_count * 16;
+    return (int)(b < 1 ? 1 : (b > cap ? cap : b));
+}
+
+int launch_fft(rtx_ctx* ctx, rtx_wave::FftArgs a, int col, long long nseq, unsigned flags) {
+    a.col = col;
+    a.flags = flags;
+    a.Ls = col ? a.L1 : a.L2;
+    a.logLs = 0;
+    while ((1 << a.logLs) < a.Ls) ++a.logLs;
+    a.C = rtx_wave::FFT_TILE / a.Ls;
+    a.nsub = nseq * (col ? a.L2 : a.L1);
+    const long long blocks = (a.nsub + a.C - 1) / a.C;
+    rtx_wave::fft_tile_kernel<<<(unsigned)blocks, rtx_wave::FFT_THREADS,
+                               rtx_wave::FFT_TILE * sizeof(double2), ctx->stream>>>(a);
+    ctx->launches++;
+    return (int)cudaGetLastError();
+}
+
+// one batch of nseq Bluestein DFTs of length M: rows of x (m_in values, stride
+// x_stride) -> rows of out (stride out_stride), epilogue `epi`
+int bluestein_rows(rtx_ctx* ctx, rtx_wave::FftArgs a, double2* work, long long work_seqs,
+                   const double2* x, long long nseq, void* out, unsigned epi) {
+    using namespace rtx_wave;
+    a.x = x;
+    if (a.L2 == 1) {  // the whole convolution in one tile
+        a.out = out;
+        return launch_fft(ctx, a, 1, nseq, F_LOAD_X | F_FWD | F_CONV | epi);
+    }
+    const size_t osz = (epi & F_OUT_ABS2) ? sizeof(double) : sizeof(double2);
+    for (long long s0 = 0; s0 < nseq; s0 += work_seqs) {
+        const long long cnt = nseq - s0 < work_seqs ? nseq - s0 : work_seqs;
+        a.x = x + s0 * a.x_stride;
+        a.work = work;
+        a.out = (char*)out + (size_t)s0 * a.out_stride * osz;
+        int rc = launch_fft(ctx, a, 1, cnt, F_LOAD_X | F_FWD | F_TWIDDLE);
+        if (!rc) rc = launch_fft(ctx, a, 0, cnt, F_FWD | F_CONV | F_TWIDDLE);
+        if (!rc) rc = launch_fft(ctx, a, 1, cnt, F_INV | epi);
+        if (rc) return rc;
+    }
+    return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rtx_opd_regrid(rtx_ctx* ctx, int64_t N, const double* A, const double* P, double a_ref,
+                   const double* p_ref, double lscale, int rings, int64_t n, double* map,
+                   double* h, int64_t* n_finite) {
+    if (!ctx || !A || !P || !p_ref || !map || rings < 1 || n < 1 || n > 46340 || lscale == 0.0)
+        return RTX_E_BADARG;
+    if (N != 1 + 3LL * rings * (rings + 1)) return RTX_E_BADARG;
+    CK(cudaSetDevice(ctx->device));
+    Scratch sc(ctx->stream);
+    unsigned long long* d_red = nullptr;  // [h bits, finite count]
+    unsigned* owner = nullptr;
+    int rc = sc.get(&d_red, 2);
+    if (!rc) rc = sc.get(&owner, (size_t)(n * n));
+    if (rc) return rc;
+    CK(cudaMemsetAsync(d_red, 0, 2 * sizeof(unsigned long long), ctx->stream));
+    CK(cudaMemsetAsync(owner, 0xff, (size_t)(n * n) * sizeof(unsigned), ctx->stream));
+    rtx_wave::RegridArgs g;
+    g.A = A;
+    g.P = P;
+    g.N = N;
+    g.ntri = 6LL * rings * rings;
+    g.a_ref = a_ref;
+    g.px_ref = p_ref[0];
+    g.py_ref = p_ref[1];
+    g.lscale = lscale;
+    g.n = (int)n;
+    g.step = n > 1 ? 2.0 / (double)(n - 1) : 1.0;  // numpy's mgrid
+    g.hbits = d_red;
+    CK(cudaEventRecord(ctx->k0, ctx->stream));
+    rtx_wave::regrid_bounds_kernel<<<grid_for(ctx, N, 256), 256, 0, ctx->stream>>>(g, d_red,
+                                                                                 d_red + 1);
+    rtx_wave::regrid_owner_kernel<<<grid_for(ctx, g.ntri, 128), 128, 0, ctx->stream>>>(g, owner);
+    rtx_wave::regrid_eval_kernel<<<grid_for(ctx, n * n, 256), 256, 0, ctx->stream>>>(g, owner,
+                                                                                   map);
+    ctx->launches += 3;
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ctx->k1, ctx->stream));
+    ctx->kernel_timed = true;
+    unsigned long long red[2];
+    CK(cudaMemcpyAsync(red, d_red, sizeof(red), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (h) memcpy(h, &red[0], sizeof(double));
+    if (n_finite) *n_finite = (int64_t)red[1];
+    return 0;
+}
+
+int rtx_psf(rtx_ctx* ctx, int64_t n, const double* map, int pad, double* psf) {
+    using namespace rtx_wave;
+    if (!ctx || !map || !psf || n < 1 || pad < 1) return RTX_E_BADARG;
+    const long long M = (long long)pad * n;
+    long long L = 1;
+    while (L < M + n - 1) L <<= 1;
+    if (L < 2) L = 2;
+    FftArgs a;
+    memset(&a, 0, sizeof(a));
+    a.L = (int)L;
+    a.L1 = L <= FFT_TILE ? (int)L : FFT_L1;
+    a.L2 = (int)(L / a.L1);
+    if (a.L2 > FFT_TILE || M > (1LL << 30) / 2) return RTX_E_UNSUPPORTED;
+    a.M = (int)M;
+    a.m_in = (int)n;
+    a.x_stride = n;
+    a.out_stride = M;
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaFuncSetAttribute(fft_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            FFT_TILE * (int)sizeof(double2)));
+    Scratch sc(ctx->stream);
+    unsigned long long* d_count = nullptr;
+    double2 *chirp = nullptr, *tw = nullptr, *bhat = nullptr, *gT = nullptr, *rows = nullptr,
+            *rowsT = nullptr, *work = nullptr;
+    // the four-step work buffer holds up to 1 GB of sequences at a time
+    const long long work_seqs = a.L2 == 1 ? 0 : ((1LL << 30) / (L * 16) > 0 ? (1LL << 30) / (L * 16)
+                                                                            : 1);
+    int rc = sc.get(&d_count, 1);
+    if (!rc) rc = sc.get(&chirp, (size_t)M);
+    if (!rc) rc = sc.get(&tw, (size_t)L);
+    if (!rc) rc = sc.get(&bhat, (size_t)L);
+    if (!rc) rc = sc.get(&gT, (size_t)(n * n));
+    if (!rc) rc = sc.get(&rows, (size_t)(n * M));
+    if (!rc) rc = sc.get(&rowsT, (size_t)(n * M));
+    if (!rc && work_seqs) rc = sc.get(&work, (size_t)(work_seqs * L));
+    if (rc) return rc;
+    a.chirp = chirp;
+    a.tw = tw;
+    a.bhat = bhat;
+    a.scale = 1.0 / ((double)M * (double)M);
+    CK(cudaEventRecord(ctx->k0, ctx->stream));
+    CK(cudaMemsetAsync(d_count, 0, sizeof(unsigned long long), ctx->stream));
+    psf_tables_kernel<<<(unsigned)((L > M ? L : M) + 255) / 256, 256, 0, ctx->stream>>>(
+        chirp, (int)M, tw, (int)L);
+    finite_count_kernel<<<grid_for(ctx, n * n, 256), 256, 0, ctx->stream>>>(map, n * n, d_count);
+    const dim3 tgrid((unsigned)((n + 31) / 32), (unsigned)((n + 31) / 32)), tblock(32, 8);
+    pupil_transpose_kernel<<<tgrid, tblock, 0, ctx->stream>>>(map, (int)n, d_count, gT);
+    ctx->launches += 3;
+    CK(cudaGetLastError());
+    // FFT_L of the Bluestein kernel, in the layout the convolution reads
+    FftArgs b = a;
+    b.work = bhat;
+    if (a.L2 == 1) {
+        rc = launch_fft(ctx, b, 1, 1, F_LOAD_B | F_FWD);
+    } else {
+        rc = launch_fft(ctx, b, 1, 1, F_LOAD_B | F_FWD | F_TWIDDLE);
+        if (!rc) rc = launch_fft(ctx, b, 0, 1, F_FWD);
+    }
+    if (rc) return rc;
+    // pass 1: the n non-zero rows of the transposed pupil -> n x M
+    rc = bluestein_rows(ctx, a, work, work_seqs, gT, n, rows, F_OUT_C);
+    if (rc) return rc;
+    transpose_kernel<<<dim3((unsigned)((M + 31) / 32), (unsigned)((n + 31) / 32)), tblock, 0,
+                       ctx->stream>>>(rows, (int)n, (int)M, rowsT);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    // pass 2: M rows of n values -> |.|^2 / M^2 into the M x M PSF
+    rc = bluestein_rows(ctx, a, work, work_seqs, rowsT, M, psf, F_OUT_ABS2);
+    if (rc) return rc;
+    CK(cudaEventRecord(ctx->k1, ctx->stream));
+    ctx->kernel_timed = true;
     return 0;
 }
 

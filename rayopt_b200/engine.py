@@ -435,6 +435,30 @@ class Engine:
             self.ctx, ptr(table), len(table), ptr(r0), _code(y0.dtype), N, y0.ptr, u0.ptr,
             int(bool(clip)), ptr(rec), A.ptr, P.ptr, self._flags(exact, False)))
 
+    def opd_regrid(self, A, P, a_ref, p_ref, lscale, rings, n, out=None):
+        """rtx_opd_regrid: the n x n OPD map (waves) of a hexapolar bundle of
+        `rings` rings from the DEVICE arrays A (N,), P (N,3) of trace_opd and
+        the reference ray's A[ref], P[ref].  Returns (map DeviceArray, h,
+        number of rays with finite x, y, t)."""
+        out = self.empty((n, n)) if out is None else out
+        h, count = C.c_double(), C.c_int64()
+        p = np.ascontiguousarray(p_ref, np.float64).reshape(3)
+        check(self.lib.rtx_opd_regrid(self.ctx, A.shape[0], A.ptr, P.ptr, float(a_ref), ptr(p),
+                                      float(lscale), int(rings), int(n), out.ptr, C.byref(h),
+                                      C.byref(count)))
+        return out, h.value, count.value
+
+    def psf(self, opd_map, pad=4, out=None):
+        """rtx_psf: the (pad n)^2 PSF of the DEVICE n x n OPD map in waves
+        (GeometricTrace.psf's definition).  Returns a DeviceArray.
+        Asynchronous."""
+        n = opd_map.shape[0]
+        if opd_map.shape != (n, n) or opd_map.dtype != np.float64:
+            raise ValueError("the OPD map must be a square float64 DeviceArray")
+        out = self.empty((pad*n, pad*n)) if out is None else out
+        check(self.lib.rtx_psf(self.ctx, n, opd_map.ptr, int(pad), out.ptr))
+        return out
+
     def ipc_export(self, darray):
         h = (C.c_ubyte*64)()
         check(self.lib.rtx_ipc_export(self.ctx, darray.ptr, C.cast(h, C.c_void_p)))

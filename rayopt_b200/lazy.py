@@ -229,6 +229,7 @@ class ResidentMixin:
         self._w_default = w is None
         self._w_dev = None
         self.ref = ref
+        self._hex_rings = None
         if width != 3:
             y0 = np.zeros((count, 3))
             u0 = np.zeros((count, 3))
@@ -361,13 +362,9 @@ class ResidentMixin:
         self.system[at].distance += shift
         return shift
 
-    def opd_rays(self, radius=None, after=-2, image=-1):
-        """per-ray part of GeometricTrace.opd (rayopt/geometric_trace.py:
-        101-131) as the epilogue of a march from row 0 to surface `after`
-        (rtx_trace_opd); the reference ray's terms are subtracted here.
-        Returns (x, y, t): exit-pupil coordinates and the OPD in waves -- what
-        ``opd(resample=False)`` returns in the reference.  Needs a propagated
-        trace (the sphere is centred on ``y[image, ref]``)."""
+    def _opd_device(self, radius=None, after=-2, image=-1):
+        """rtx_trace_opd into fresh DEVICE arrays A (N,), P (N,3); returns them
+        with the reference ray's A[ref], P[ref] and l/scale"""
         eng, s, d = self._engine(), self.system, self._dev
         after, image = range(self.length)[after], range(self.length)[image]
         ref = int(self.ref)
@@ -390,11 +387,23 @@ class ResidentMixin:
         A, P = eng.empty((self.nrays,)), eng.empty((self.nrays, 3))
         eng.trace_opd(table, d["y"].rows(0), d["u"].rows(0), spec, A, P, N=self.nrays,
                       clip=getattr(self, "_last_clip", False), rot0=rot0, exact=self.exact)
+        a_ref = A.rows(ref).download()[0]
+        p_ref = eng.download_rays(P, [ref])[0]
+        return A, P, a_ref, p_ref, self.l/s.scale
+
+    def opd_rays(self, radius=None, after=-2, image=-1):
+        """per-ray part of GeometricTrace.opd (rayopt/geometric_trace.py:
+        101-131) as the epilogue of a march from row 0 to surface `after`
+        (rtx_trace_opd); the reference ray's terms are subtracted here.
+        Returns (x, y, t): exit-pupil coordinates and the OPD in waves -- what
+        ``opd(resample=False)`` returns in the reference.  Needs a propagated
+        trace (the sphere is centred on ``y[image, ref]``)."""
+        A, P, a_ref, p_ref, lscale = self._opd_device(radius, after, image)
         a, p = A.download(), P.download()
         A.free()
         P.free()
-        t = -(a - a[ref])/(self.l/s.scale)                  # :125-126
-        p -= p[ref]                                         # :131
+        t = -(a - a_ref)/lscale                             # :125-126
+        p -= p_ref                                          # :131
         return p[:, 0], p[:, 1], t
 
     def opd(self, radius=None, after=-2, image=-1, resample=4):
@@ -413,6 +422,91 @@ class ResidentMixin:
             t = griddata((x, y), t, (xs, ys), method="linear", fill_value=np.nan)
             x, y = xs, ys
         return x, y, t
+
+    # ---- the OPD map and the PSF in HBM (rtx_opd_regrid, rtx_psf)
+    # rings of the hexapolar launch grid when the launch rays are known to be
+    # pupil_distribution("hexapolar") without a pupil filter, else None: the
+    # ray index then gives the triangulation (rtx_opd_regrid)
+    _hex_rings = None
+
+    def rays_point(self, yo, wavelength=None, nrays=11, distribution="meridional", filter=None,
+                   stop=None, clip=False):
+        """GeometricTrace.rays_point (rayopt/geometric_trace.py:204-209) of the
+        reference, recording whether the bundle is an unfiltered hexapolar
+        grid (its `filter` defaults to ``not clip``)"""
+        super().rays_point(yo, wavelength, nrays, distribution, filter, stop, clip)
+        self._record_grid(distribution, nrays, (not clip) if filter is None else filter)
+
+    def _record_grid(self, distribution, nrays, filter):
+        rings = int(np.sqrt(nrays/3. - 1/12.) - 1/2.) if distribution == "hexapolar" else 0
+        ok = int(nrays) > 1 and not filter and rings >= 1 and self.nrays == 1 + 3*rings*(rings + 1)
+        self._hex_rings = rings if ok else None
+
+    def _opd_grid(self, radius, after, image, resample, regrid):
+        """(map, h, x): the (n, n) OPD map in HBM, h (None for the host path)
+        and the x column of the node grid; regridded on the device, or by
+        scipy griddata on the host (opd()) and uploaded"""
+        if regrid is None:
+            regrid = "host" if self._hex_rings is None else "device"
+        if regrid == "host":
+            xs, _, t = self.opd(radius, after, image, resample)
+            return self._engine().to_device(t), None, xs[:, 0]
+        if regrid != "device":
+            raise ValueError("regrid must be 'device', 'host' or None, got %r" % (regrid,))
+        if self._hex_rings is None:
+            raise ValueError("device regridding needs a hexapolar bundle generated without "
+                             "a pupil filter (rays_point(distribution='hexapolar', clip=True))")
+        A, P, a_ref, p_ref, lscale = self._opd_device(radius, after, image)
+        n = int(resample*self.nrays**.5)
+        try:
+            m, h, count = self._engine().opd_regrid(A, P, a_ref, p_ref, lscale, self._hex_rings, n)
+        finally:
+            A.free()
+            P.free()
+        if not count:
+            m.free()
+            raise ValueError("no rays made it through")
+        return m, h, np.mgrid[-1:1:1j*n, -1:1:2j][0][:, 0]*h
+
+    def opd_map(self, radius=None, after=-2, image=-1, resample=4, regrid=None):
+        """GeometricTrace.opd(resample) (rayopt/geometric_trace.py:101-144):
+        returns the reference's (x, y, t) node grids.  regrid="device"
+        interpolates on the structured triangulation of a hexapolar launch
+        grid in HBM (rtx_opd_regrid; vignetted gaps stay NaN, INTEGRATION.md
+        section 5), "host" is opd(); None picks "device" when the bundle is
+        known to be an unfiltered hexapolar grid."""
+        if not resample or regrid == "host" or (regrid is None and self._hex_rings is None):
+            return self.opd(radius, after, image, resample)
+        m, h, _ = self._opd_grid(radius, after, image, resample, regrid)
+        t = m.download()
+        m.free()
+        n = t.shape[0]
+        xs, ys = np.mgrid[-1:1:1j*n, -1:1:1j*n]*h
+        return xs, ys, t
+
+    def psf_device(self, pad=4, resample=4, regrid=None, **kw):
+        """GeometricTrace.psf (rayopt/geometric_trace.py:146-169) with the
+        pupil function, the zero-padded 2-D DFT and |.|^2 in HBM (rtx_psf);
+        the OPD map comes from opd_map's `regrid`.  Returns (p, q, psf)."""
+        radius = self.system[-1].distance                   # :147
+        m, _, x = self._opd_grid(radius, kw.pop("after", -2), kw.pop("image", -1), resample,
+                                 regrid)
+        if kw:
+            raise TypeError("unexpected arguments %s" % sorted(kw))
+        eng = self._engine()
+        n = m.shape[0]
+        try:
+            d_psf = eng.psf(m, pad)
+        finally:
+            m.free()
+        psf = eng.pinned_empty(d_psf.shape) if d_psf.nbytes >= PINNED_ROW_BYTES else None
+        psf = d_psf.download(psf)
+        d_psf.free()
+        dx = x[1] - x[0]                                    # :158-161
+        k = 1/(self.l/self.system.scale)
+        f = np.fft.fftfreq(pad*n, dx*k/radius)
+        p, q = np.broadcast_arrays(f[:, None], f)
+        return p, q, psf
 
 
 class ResidentTrace(ResidentMixin):
@@ -449,6 +543,7 @@ class ResidentTrace(ResidentMixin):
         pmax = float(np.fabs(np.asarray(p, float)).max())
         d = self._dev
         eng.aim_infinite_into(d["y"].rows(0), d["u"].rows(0), count, rings, frame, pmax, yp)
+        self._hex_rings = rings if yp is None and rings >= 1 else None
         d["i"].rows(0).copy_from(d["u"].rows(0), count*24)   # i[0] = u[0] (geometric_trace.py:68)
         self._zero_t0()
         for a in (self.y, self.u, self.i, self.t):
@@ -481,6 +576,7 @@ class ResidentTrace(ResidentMixin):
         self.ref = ref
         d = self._dev
         eng.aim_rays_into(spec, d["y"].rows(0), d["u"].rows(0), count)
+        self._record_grid(distribution, nrays, filter)
         d["i"].rows(0).copy_from(d["u"].rows(0), count*24)   # i[0] = u[0] (geometric_trace.py:68)
         self._zero_t0()
         for a in (self.y, self.u, self.i, self.t):
