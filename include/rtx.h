@@ -513,6 +513,48 @@ int rtx_opd_regrid(rtx_ctx *ctx, int64_t N, const double *A, const double *P,
  */
 int rtx_psf(rtx_ctx *ctx, int64_t n, const double *map, int pad, double *psf);
 
+/* ---- PSF figures (rayopt/analysis.py:319-346, Analysis.opds) ------------- */
+/*
+ * On the UNSHIFTED M x M FP64 PSF in DEVICE memory, as rtx_psf writes it
+ * (1 <= M <= RTX_PSF_MAX_M).  fftshift maps unshifted index i to shifted
+ * index (i + M/2) % M.  Every result is bit-identical run to run.
+ */
+#define RTX_PSF_MAX_M 1048576
+
+/*
+ * One read of psf: DEVICE lines (2, M) = psf.sum(0), then psf.sum(1), each
+ * sum in a fixed order; HOST stats[3] = max element, sum of all elements,
+ * and the count of elements that are non-finite or outside [0, 2].
+ * Synchronises.
+ */
+int rtx_psf_lines(rtx_ctx *ctx, int64_t M, const double *psf, double *lines,
+                  double *stats);
+
+/*
+ * special_sums.polar_sum(fftshift(psf), (c0, c1), "azimuthal") in fixed
+ * point: shifted node (I, J) falls in bin trunc(sqrt((J - c1)^2 + (I - c0)^2))
+ * (unfused IEEE in that order) and adds rint(psf * 2^62) to HOST bins
+ * (nbins uint64).  Integer sums do not depend on the order of the atomics.
+ * Needs every element in [0, 2] and their sum <= 2 (rtx_psf_lines checks
+ * both).  RTX_E_BADARG when an element's bin is >= nbins.  Synchronises.
+ */
+int rtx_psf_encircled(rtx_ctx *ctx, int64_t M, const double *psf, double c0,
+                      double c1, int64_t nbins, uint64_t *bins);
+
+/*
+ * |DFT_M| of the two DEVICE lines (2, M) into DEVICE mtf (2, M/2): the first
+ * M/2 frequencies of each, with the library's Bluestein FFT (M >= 2).
+ * Asynchronous on the context stream.
+ */
+int rtx_psf_mtf(rtx_ctx *ctx, int64_t M, const double *lines, double *mtf);
+
+/*
+ * DEVICE out (w, w) = fftshift(psf)[(i0 + a) % M, (j0 + b) % M], indices
+ * taken modulo M (1 <= w <= M).  Asynchronous on the context stream.
+ */
+int rtx_psf_window(rtx_ctx *ctx, int64_t M, const double *psf, int64_t i0,
+                   int64_t j0, int64_t w, double *out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -71,6 +71,10 @@ SYMBOLS = {
     "rtx_opd_regrid": (_i, [_vp, _i64, _vp, _vp, C.c_double, _vp, C.c_double, _i, _i64, _vp,
                             _vp, _vp]),
     "rtx_psf": (_i, [_vp, _i64, _vp, _i, _vp]),
+    "rtx_psf_lines": (_i, [_vp, _i64, _vp, _vp, _vp]),
+    "rtx_psf_encircled": (_i, [_vp, _i64, _vp, C.c_double, C.c_double, _i64, _vp]),
+    "rtx_psf_mtf": (_i, [_vp, _i64, _vp, _vp]),
+    "rtx_psf_window": (_i, [_vp, _i64, _vp, _i64, _i64, _i64, _vp]),
 }
 
 _lib = None

@@ -1774,6 +1774,56 @@ int bluestein_rows(rtx_ctx* ctx, rtx_wave::FftArgs a, double2* work, long long w
     return 0;
 }
 
+// length-M DFTs of rows of m_in values as Bluestein convolutions: L, the
+// four-step split and the lengths in `a` (zeroed first)
+int bluestein_plan(long long M, long long m_in, rtx_wave::FftArgs& a) {
+    using namespace rtx_wave;
+    long long L = 1;
+    while (L < M + m_in - 1) L <<= 1;
+    if (L < 2) L = 2;
+    memset(&a, 0, sizeof(a));
+    a.L = (int)L;
+    a.L1 = L <= FFT_TILE ? (int)L : FFT_L1;
+    a.L2 = (int)(L / a.L1);
+    if (a.L2 > FFT_TILE || M > (1LL << 30) / 2) return RTX_E_UNSUPPORTED;
+    a.M = (int)M;
+    a.m_in = (int)m_in;
+    return 0;
+}
+
+// sequences the four-step work buffer holds (up to 1 GB); 0 in one tile
+long long bluestein_work_seqs(const rtx_wave::FftArgs& a) {
+    if (a.L2 == 1) return 0;
+    const long long s = (1LL << 30) / ((long long)a.L * 16);
+    return s > 0 ? s : 1;
+}
+
+// the chirp and twiddle tables and FFT_L of the Bluestein kernel, in the
+// layout the convolution reads, into scratch of `sc`; enqueued on the stream
+int bluestein_tables(rtx_ctx* ctx, Scratch& sc, rtx_wave::FftArgs& a) {
+    using namespace rtx_wave;
+    CK(cudaFuncSetAttribute(fft_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            FFT_TILE * (int)sizeof(double2)));
+    double2 *chirp = nullptr, *tw = nullptr, *bhat = nullptr;
+    int rc = sc.get(&chirp, (size_t)a.M);
+    if (!rc) rc = sc.get(&tw, (size_t)a.L);
+    if (!rc) rc = sc.get(&bhat, (size_t)a.L);
+    if (rc) return rc;
+    a.chirp = chirp;
+    a.tw = tw;
+    a.bhat = bhat;
+    psf_tables_kernel<<<(unsigned)((a.L > a.M ? a.L : a.M) + 255) / 256, 256, 0, ctx->stream>>>(
+        chirp, a.M, tw, a.L);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    FftArgs b = a;
+    b.work = bhat;
+    if (a.L2 == 1) return launch_fft(ctx, b, 1, 1, F_LOAD_B | F_FWD);
+    rc = launch_fft(ctx, b, 1, 1, F_LOAD_B | F_FWD | F_TWIDDLE);
+    if (!rc) rc = launch_fft(ctx, b, 0, 1, F_FWD);
+    return rc;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1827,61 +1877,32 @@ int rtx_psf(rtx_ctx* ctx, int64_t n, const double* map, int pad, double* psf) {
     using namespace rtx_wave;
     if (!ctx || !map || !psf || n < 1 || pad < 1) return RTX_E_BADARG;
     const long long M = (long long)pad * n;
-    long long L = 1;
-    while (L < M + n - 1) L <<= 1;
-    if (L < 2) L = 2;
     FftArgs a;
-    memset(&a, 0, sizeof(a));
-    a.L = (int)L;
-    a.L1 = L <= FFT_TILE ? (int)L : FFT_L1;
-    a.L2 = (int)(L / a.L1);
-    if (a.L2 > FFT_TILE || M > (1LL << 30) / 2) return RTX_E_UNSUPPORTED;
-    a.M = (int)M;
-    a.m_in = (int)n;
+    int rc = bluestein_plan(M, n, a);
+    if (rc) return rc;
     a.x_stride = n;
     a.out_stride = M;
     CK(cudaSetDevice(ctx->device));
-    CK(cudaFuncSetAttribute(fft_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            FFT_TILE * (int)sizeof(double2)));
     Scratch sc(ctx->stream);
     unsigned long long* d_count = nullptr;
-    double2 *chirp = nullptr, *tw = nullptr, *bhat = nullptr, *gT = nullptr, *rows = nullptr,
-            *rowsT = nullptr, *work = nullptr;
-    // the four-step work buffer holds up to 1 GB of sequences at a time
-    const long long work_seqs = a.L2 == 1 ? 0 : ((1LL << 30) / (L * 16) > 0 ? (1LL << 30) / (L * 16)
-                                                                            : 1);
-    int rc = sc.get(&d_count, 1);
-    if (!rc) rc = sc.get(&chirp, (size_t)M);
-    if (!rc) rc = sc.get(&tw, (size_t)L);
-    if (!rc) rc = sc.get(&bhat, (size_t)L);
+    double2 *gT = nullptr, *rows = nullptr, *rowsT = nullptr, *work = nullptr;
+    const long long work_seqs = bluestein_work_seqs(a);
+    rc = sc.get(&d_count, 1);
     if (!rc) rc = sc.get(&gT, (size_t)(n * n));
     if (!rc) rc = sc.get(&rows, (size_t)(n * M));
     if (!rc) rc = sc.get(&rowsT, (size_t)(n * M));
-    if (!rc && work_seqs) rc = sc.get(&work, (size_t)(work_seqs * L));
+    if (!rc && work_seqs) rc = sc.get(&work, (size_t)(work_seqs * a.L));
     if (rc) return rc;
-    a.chirp = chirp;
-    a.tw = tw;
-    a.bhat = bhat;
     a.scale = 1.0 / ((double)M * (double)M);
     CK(cudaEventRecord(ctx->k0, ctx->stream));
     CK(cudaMemsetAsync(d_count, 0, sizeof(unsigned long long), ctx->stream));
-    psf_tables_kernel<<<(unsigned)((L > M ? L : M) + 255) / 256, 256, 0, ctx->stream>>>(
-        chirp, (int)M, tw, (int)L);
+    rc = bluestein_tables(ctx, sc, a);
+    if (rc) return rc;
     finite_count_kernel<<<grid_for(ctx, n * n, 256), 256, 0, ctx->stream>>>(map, n * n, d_count);
     const dim3 tgrid((unsigned)((n + 31) / 32), (unsigned)((n + 31) / 32)), tblock(32, 8);
     pupil_transpose_kernel<<<tgrid, tblock, 0, ctx->stream>>>(map, (int)n, d_count, gT);
-    ctx->launches += 3;
+    ctx->launches += 2;
     CK(cudaGetLastError());
-    // FFT_L of the Bluestein kernel, in the layout the convolution reads
-    FftArgs b = a;
-    b.work = bhat;
-    if (a.L2 == 1) {
-        rc = launch_fft(ctx, b, 1, 1, F_LOAD_B | F_FWD);
-    } else {
-        rc = launch_fft(ctx, b, 1, 1, F_LOAD_B | F_FWD | F_TWIDDLE);
-        if (!rc) rc = launch_fft(ctx, b, 0, 1, F_FWD);
-    }
-    if (rc) return rc;
     // pass 1: the n non-zero rows of the transposed pupil -> n x M
     rc = bluestein_rows(ctx, a, work, work_seqs, gT, n, rows, F_OUT_C);
     if (rc) return rc;
@@ -1894,6 +1915,120 @@ int rtx_psf(rtx_ctx* ctx, int64_t n, const double* map, int pad, double* psf) {
     if (rc) return rc;
     CK(cudaEventRecord(ctx->k1, ctx->stream));
     ctx->kernel_timed = true;
+    return 0;
+}
+
+int rtx_psf_lines(rtx_ctx* ctx, int64_t M, const double* psf, double* lines, double* stats) {
+    using namespace rtx_wave;
+    if (!ctx || !psf || !lines || !stats || M < 1 || M > RTX_PSF_MAX_M) return RTX_E_BADARG;
+    CK(cudaSetDevice(ctx->device));
+    const int nchunk = (int)((M + LINES_CW - 1) / LINES_CW);
+    const int nband = (int)((M + LINES_RB - 1) / LINES_RB);
+    const long long nblocks = (long long)nchunk * nband;
+    Scratch sc(ctx->stream);
+    double *colp = nullptr, *rowp = nullptr, *bmax = nullptr, *d_stats = nullptr;
+    unsigned long long* bbad = nullptr;
+    int rc = sc.get(&colp, (size_t)(nband * M));
+    if (!rc) rc = sc.get(&rowp, (size_t)(nchunk * M));
+    if (!rc) rc = sc.get(&bmax, (size_t)nblocks);
+    if (!rc) rc = sc.get(&bbad, (size_t)nblocks);
+    if (!rc) rc = sc.get(&d_stats, 3);
+    if (rc) return rc;
+    CK(cudaEventRecord(ctx->k0, ctx->stream));
+    psf_lines_tile_kernel<<<dim3((unsigned)nchunk, (unsigned)nband), LINES_THREADS, 0,
+                            ctx->stream>>>(psf, (int)M, colp, rowp, bmax, bbad);
+    psf_lines_finish_kernel<<<(unsigned)((M + 255) / 256), 256, 0, ctx->stream>>>(
+        colp, rowp, (int)M, nband, nchunk, lines);
+    psf_stats_kernel<<<1, LINES_THREADS, 0, ctx->stream>>>(lines + M, (int)M, bmax, bbad,
+                                                          nblocks, d_stats);
+    ctx->launches += 3;
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ctx->k1, ctx->stream));
+    ctx->kernel_timed = true;
+    CK(cudaMemcpyAsync(stats, d_stats, 3 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+int rtx_psf_encircled(rtx_ctx* ctx, int64_t M, const double* psf, double c0, double c1,
+                      int64_t nbins, uint64_t* bins) {
+    using namespace rtx_wave;
+    if (!ctx || !psf || !bins || M < 1 || M > RTX_PSF_MAX_M || nbins < 1 || !std::isfinite(c0) ||
+        !std::isfinite(c1))
+        return RTX_E_BADARG;
+    CK(cudaSetDevice(ctx->device));
+    Scratch sc(ctx->stream);
+    unsigned long long* d_bins = nullptr;
+    int* d_over = nullptr;
+    int rc = sc.get(&d_bins, (size_t)nbins);
+    if (!rc) rc = sc.get(&d_over, 1);
+    if (rc) return rc;
+    CK(cudaMemsetAsync(d_bins, 0, (size_t)nbins * sizeof(unsigned long long), ctx->stream));
+    CK(cudaMemsetAsync(d_over, 0, sizeof(int), ctx->stream));
+    const unsigned tiles = (unsigned)((M + EE_T - 1) / EE_T);
+    CK(cudaEventRecord(ctx->k0, ctx->stream));
+    psf_encircled_kernel<<<dim3(tiles, tiles), EE_THREADS, 0, ctx->stream>>>(
+        psf, (int)M, c0, c1, nbins, d_bins, d_over);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ctx->k1, ctx->stream));
+    ctx->kernel_timed = true;
+    int over = 0;
+    CK(cudaMemcpyAsync(bins, d_bins, (size_t)nbins * sizeof(unsigned long long),
+                       cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&over, d_over, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return over ? RTX_E_BADARG : 0;
+}
+
+int rtx_psf_mtf(rtx_ctx* ctx, int64_t M, const double* lines, double* mtf) {
+    using namespace rtx_wave;
+    if (!ctx || !lines || !mtf || M < 2 || M > RTX_PSF_MAX_M) return RTX_E_BADARG;
+    FftArgs a;
+    int rc = bluestein_plan(M, M, a);
+    if (rc) return rc;
+    a.x_stride = M;
+    a.out_stride = M;
+    a.scale = 1.0;
+    CK(cudaSetDevice(ctx->device));
+    Scratch sc(ctx->stream);
+    double2 *z = nullptr, *work = nullptr;
+    double* abs2 = nullptr;
+    const long long work_seqs = bluestein_work_seqs(a);
+    rc = sc.get(&z, (size_t)(2 * M));
+    if (!rc) rc = sc.get(&abs2, (size_t)(2 * M));
+    if (!rc && work_seqs) rc = sc.get(&work, (size_t)(work_seqs * a.L));
+    if (rc) return rc;
+    CK(cudaEventRecord(ctx->k0, ctx->stream));
+    rc = bluestein_tables(ctx, sc, a);
+    if (rc) return rc;
+    real_to_complex_kernel<<<(unsigned)((2 * M + 255) / 256), 256, 0, ctx->stream>>>(lines, 2 * M,
+                                                                                   z);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    rc = bluestein_rows(ctx, a, work, work_seqs, z, 2, abs2, F_OUT_ABS2);
+    if (rc) return rc;
+    const int half = (int)(M / 2);
+    psf_abs_half_kernel<<<(unsigned)((2 * half + 255) / 256), 256, 0, ctx->stream>>>(
+        abs2, (int)M, half, 2, mtf);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ctx->k1, ctx->stream));
+    ctx->kernel_timed = true;
+    return 0;
+}
+
+int rtx_psf_window(rtx_ctx* ctx, int64_t M, const double* psf, int64_t i0, int64_t j0, int64_t w,
+                   double* out) {
+    using namespace rtx_wave;
+    if (!ctx || !psf || !out || M < 1 || M > RTX_PSF_MAX_M || w < 1 || w > M) return RTX_E_BADARG;
+    CK(cudaSetDevice(ctx->device));
+    const int i = (int)(((i0 % M) + M) % M), j = (int)(((j0 % M) + M) % M);
+    psf_window_kernel<<<dim3((unsigned)((w + 127) / 128), (unsigned)(w < 65535 ? w : 65535)), 128,
+                        0, ctx->stream>>>(
+        psf, (int)M, i, j, (int)w, out);
+    ctx->launches++;
+    CK(cudaGetLastError());
     return 0;
 }
 

@@ -414,4 +414,222 @@ __global__ void transpose_kernel(const double2* in, int rows, int cols, double2*
     }
 }
 
+// ---- PSF figures (Analysis.opds, rayopt/analysis.py:319-346) -----------------
+//
+// All on the UNSHIFTED M x M PSF of rtx_psf.  Line sums: psf.sum(0) (per
+// column) and psf.sum(1) (per row) from one read, in a fixed reduction order.
+// Encircled energy: a radial histogram in the fftshifted frame (shifted index
+// I = (i + M/2) % M), bin trunc(sqrt((J - c1)^2 + (I - c0)^2)) in unfused IEEE,
+// accumulated in 2^-62 fixed point so that the sum is exact integer arithmetic
+// and independent of the atomic order.
+
+constexpr int LINES_THREADS = 256;
+constexpr int LINES_PER_THREAD = 4;                            // columns per thread
+constexpr int LINES_CW = LINES_THREADS * LINES_PER_THREAD;     // columns per tile
+constexpr int LINES_RB = 128;                                  // rows per tile
+
+// one RB x CW tile per CTA: column partials colp[band][j], row partials
+// rowp[chunk][i], and per-CTA max and count of elements that are non-finite or
+// outside [0, 2]
+__global__ void __launch_bounds__(LINES_THREADS)
+    psf_lines_tile_kernel(const double* psf, int M, double* colp, double* rowp, double* bmax,
+                          unsigned long long* bbad) {
+    __shared__ double wsum[LINES_RB][LINES_THREADS / 32];
+    __shared__ double smax[LINES_THREADS / 32];
+    __shared__ unsigned long long sbad[LINES_THREADS / 32];
+    const int band = blockIdx.y, chunk = blockIdx.x;
+    const int i0 = band * LINES_RB, j0 = chunk * LINES_CW;
+    const int rows = min(LINES_RB, M - i0);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double col[LINES_PER_THREAD];
+    for (int k = 0; k < LINES_PER_THREAD; ++k) col[k] = 0.0;
+    double mx = 0.0;
+    unsigned long long bad = 0;
+#pragma unroll 4
+    for (int r = 0; r < rows; ++r) {
+        const double* row = psf + (long long)(i0 + r) * M;
+        double v[LINES_PER_THREAD];
+#pragma unroll
+        for (int k = 0; k < LINES_PER_THREAD; ++k) {
+            const int j = j0 + threadIdx.x + k * LINES_THREADS;
+            v[k] = j < M ? __ldcs(row + j) : 0.0;
+        }
+        double s = 0.0;
+#pragma unroll
+        for (int k = 0; k < LINES_PER_THREAD; ++k) {
+            col[k] = __dadd_rn(col[k], v[k]);
+            s = __dadd_rn(s, v[k]);
+            mx = fmax(mx, v[k]);
+            bad += (v[k] >= 0.0 && v[k] <= 2.0) ? 0 : 1;  // NaN fails both
+        }
+        for (int o = 16; o; o >>= 1) s = __dadd_rn(s, __shfl_xor_sync(0xffffffffu, s, o));
+        if (lane == 0) wsum[r][warp] = s;
+    }
+#pragma unroll
+    for (int k = 0; k < LINES_PER_THREAD; ++k) {
+        const int j = j0 + threadIdx.x + k * LINES_THREADS;
+        if (j < M) colp[(long long)band * M + j] = col[k];
+    }
+    for (int o = 16; o; o >>= 1) {
+        mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+        bad += __shfl_xor_sync(0xffffffffu, bad, o);
+    }
+    if (lane == 0) {
+        smax[warp] = mx;
+        sbad[warp] = bad;
+    }
+    __syncthreads();
+    if (threadIdx.x < rows) {
+        double s = 0.0;
+        for (int w = 0; w < LINES_THREADS / 32; ++w) s = __dadd_rn(s, wsum[threadIdx.x][w]);
+        rowp[(long long)chunk * M + i0 + threadIdx.x] = s;
+    }
+    if (threadIdx.x == 0) {
+        for (int w = 0; w < LINES_THREADS / 32; ++w) {
+            mx = fmax(mx, smax[w]);
+            bad += w ? sbad[w] : 0;
+        }
+        const long long b = (long long)band * gridDim.x + chunk;
+        bmax[b] = mx;
+        bbad[b] = bad;
+    }
+}
+
+// lines[j] = sum over bands of colp[band][j], lines[M + i] = sum over chunks of
+// rowp[chunk][i], each in index order
+__global__ void psf_lines_finish_kernel(const double* colp, const double* rowp, int M, int nband,
+                                        int nchunk, double* lines) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= M) return;
+    double c = 0.0, r = 0.0;
+    for (int b = 0; b < nband; ++b) c = __dadd_rn(c, colp[(long long)b * M + j]);
+    for (int b = 0; b < nchunk; ++b) r = __dadd_rn(r, rowp[(long long)b * M + j]);
+    lines[j] = c;
+    lines[M + j] = r;
+}
+
+// stats = (max over CTAs, sum of the row sums, count of bad elements); one CTA
+// of LINES_THREADS threads, fixed strides and a fixed tree
+__global__ void __launch_bounds__(LINES_THREADS)
+    psf_stats_kernel(const double* rows, int M, const double* bmax,
+                     const unsigned long long* bbad, long long nblocks, double* stats) {
+    __shared__ double ssum[LINES_THREADS], smax[LINES_THREADS];
+    __shared__ unsigned long long sbad[LINES_THREADS];
+    double s = 0.0, mx = 0.0;
+    unsigned long long bad = 0;
+    for (int i = threadIdx.x; i < M; i += LINES_THREADS) s = __dadd_rn(s, rows[i]);
+    for (long long b = threadIdx.x; b < nblocks; b += LINES_THREADS) {
+        mx = fmax(mx, bmax[b]);
+        bad += bbad[b];
+    }
+    ssum[threadIdx.x] = s;
+    smax[threadIdx.x] = mx;
+    sbad[threadIdx.x] = bad;
+    __syncthreads();
+    for (int h = LINES_THREADS / 2; h; h >>= 1) {
+        if (threadIdx.x < h) {
+            ssum[threadIdx.x] = __dadd_rn(ssum[threadIdx.x], ssum[threadIdx.x + h]);
+            smax[threadIdx.x] = fmax(smax[threadIdx.x], smax[threadIdx.x + h]);
+            sbad[threadIdx.x] += sbad[threadIdx.x + h];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        stats[0] = smax[0];
+        stats[1] = ssum[0];
+        stats[2] = (double)sbad[0];
+    }
+}
+
+constexpr int EE_THREADS = 256;
+constexpr int EE_T = 128;     // EE_T x EE_T shifted-frame tile per CTA
+constexpr int EE_HB = 256;    // shared bins per CTA: a tile spans <= sqrt(2) EE_T + 2 bins
+constexpr double EE_ONE = 0x1p62;
+
+// the bin of shifted node (I, J): polar_sum's (j**2 + i**2)**.5, truncated
+__device__ __forceinline__ long long ee_bin(int I, int J, double c0, double c1) {
+    const double di = __dsub_rn((double)I, c0), dj = __dsub_rn((double)J, c1);
+    return (long long)__dsqrt_rn(__dadd_rn(__dmul_rn(dj, dj), __dmul_rn(di, di)));
+}
+
+// distance from c to the nearest node of [lo, hi]
+__device__ __forceinline__ double ee_near(int lo, int hi, double c) {
+    return c < lo ? lo - c : (c > hi ? c - hi : 0.0);
+}
+
+__global__ void __launch_bounds__(EE_THREADS)
+    psf_encircled_kernel(const double* psf, int M, double c0, double c1, long long nbins,
+                         unsigned long long* bins, int* overflow) {
+    __shared__ unsigned long long hist[EE_HB];
+    const int I0 = blockIdx.y * EE_T, J0 = blockIdx.x * EE_T;
+    const int I1 = min(I0 + EE_T, M) - 1, J1 = min(J0 + EE_T, M) - 1;
+    // lowest bin of the tile, less a margin; elements outside the shared range
+    // go straight to global memory
+    const double di = ee_near(I0, I1, c0), dj = ee_near(J0, J1, c1);
+    const long long lo = max(0LL, (long long)sqrt(dj * dj + di * di) - 2);
+    for (int b = threadIdx.x; b < EE_HB; b += EE_THREADS) hist[b] = 0;
+    __syncthreads();
+    const int h = M / 2;
+    const int J = J0 + (threadIdx.x % EE_T);
+    const int j = J - h < 0 ? J - h + M : J - h;  // unshifted column
+    constexpr int STEP = EE_THREADS / EE_T, U = 4;  // U rows loaded before any atomic
+    if (J <= J1) {
+        for (int Ib = I0 + threadIdx.x / EE_T; Ib <= I1; Ib += STEP * U) {
+            double v[U];
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                const int I = Ib + u * STEP;
+                const int i = I - h < 0 ? I - h + M : I - h;
+                v[u] = I <= I1 ? __ldcs(psf + (long long)i * M + j) : 0.0;
+            }
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                const unsigned long long q = __double2ull_rn(__dmul_rn(v[u], EE_ONE));
+                if (!q) continue;
+                const long long b = ee_bin(Ib + u * STEP, J, c0, c1);
+                if (b >= nbins) {
+                    atomicOr(overflow, 1);
+                } else if (b >= lo && b < lo + EE_HB) {
+                    atomicAdd(&hist[b - lo], q);
+                } else {
+                    atomicAdd(&bins[b], q);
+                }
+            }
+        }
+    }
+    __syncthreads();
+    for (int b = threadIdx.x; b < EE_HB; b += EE_THREADS)
+        if (hist[b]) atomicAdd(&bins[lo + b], hist[b]);
+}
+
+// |X| = sqrt(|X|^2) of the first `half` of each of `nseq` rows of M values
+__global__ void psf_abs_half_kernel(const double* abs2, int M, int half, int nseq, double* out) {
+    const long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (k >= (long long)half * nseq) return;
+    const long long s = k / half, e = k - s * half;
+    out[k] = sqrt(abs2[s * M + e]);
+}
+
+// real rows -> complex rows (imaginary part 0)
+__global__ void real_to_complex_kernel(const double* x, long long n, double2* z) {
+    const long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (k < n) z[k] = make_double2(x[k], 0.0);
+}
+
+// out[a][b] = fftshift(psf)[(i0 + a) % M][(j0 + b) % M], 0 <= i0, j0 < M
+__global__ void psf_window_kernel(const double* psf, int M, int i0, int j0, int w, double* out) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= w) return;
+    const int h = M / 2;
+    int J = j0 + b;
+    J -= J >= M ? M : 0;
+    const int j = J - h < 0 ? J - h + M : J - h;
+    for (int a = blockIdx.y; a < w; a += gridDim.y) {
+        int I = i0 + a;
+        I -= I >= M ? M : 0;
+        const int i = I - h < 0 ? I - h + M : I - h;
+        out[(long long)a * w + b] = psf[(long long)i * M + j];
+    }
+}
+
 }  // namespace rtx_wave

@@ -5,7 +5,9 @@ the trace call with host or device buffers, CUDA-event timing.  One `Engine`
 per GPU (one process per GPU in multi-GPU runs).
 """
 import ctypes as C
+import math
 import weakref
+from collections import namedtuple
 
 import numpy as np
 
@@ -20,6 +22,9 @@ _DTYPES = {np.dtype(np.float64): RTX_F64, np.dtype(np.float32): RTX_F32}
 OPD_DTYPE = np.dtype([("y0_ref", "<f8", (3,)), ("u0_ref", "<f8", (3,)), ("n0", "<f8"),
                       ("n_after", "<f8"), ("M", "<f8", (9,)), ("d", "<f8", (3,)),
                       ("radius", "<f8"), ("infinite", "<i4"), ("reserved", "<i4")], align=True)
+
+# the figures of a PSF (Engine.psf_metrics)
+PsfMetrics = namedtuple("PsfMetrics", "x0 y0 dx peak ee r freq mtf window")
 
 
 def _code(dtype):
@@ -458,6 +463,116 @@ class Engine:
         out = self.empty((pad*n, pad*n)) if out is None else out
         check(self.lib.rtx_psf(self.ctx, n, opd_map.ptr, int(pad), out.ptr))
         return out
+
+    @staticmethod
+    def _square(d_psf):
+        M = d_psf.shape[0]
+        if d_psf.shape != (M, M) or d_psf.dtype != np.float64:
+            raise ValueError("the PSF must be a square float64 DeviceArray")
+        return M
+
+    def psf_lines(self, d_psf, out=None):
+        """rtx_psf_lines: one read of the DEVICE (M, M) PSF.  Returns (lines
+        DeviceArray (2, M) = psf.sum(0), psf.sum(1); peak; total; number of
+        elements that are non-finite or outside [0, 2])."""
+        M = self._square(d_psf)
+        out = self.empty((2, M)) if out is None else out
+        stats = (C.c_double*3)()
+        check(self.lib.rtx_psf_lines(self.ctx, M, d_psf.ptr, out.ptr, stats))
+        return out, stats[0], stats[1], int(stats[2])
+
+    def psf_encircled(self, d_psf, c0, c1, nbins):
+        """rtx_psf_encircled: the radial histogram of fftshift(psf) about the
+        shifted-frame center (c0, c1) in units of 2^-62 (uint64, nbins)"""
+        M = self._square(d_psf)
+        bins = np.empty(int(nbins), np.uint64)
+        rc = self.lib.rtx_psf_encircled(self.ctx, M, d_psf.ptr, float(c0), float(c1), int(nbins),
+                                        ptr(bins))
+        if rc == -1:
+            raise ValueError("an element's bin is beyond nbins = %d" % nbins)
+        check(rc)
+        return bins
+
+    def psf_mtf(self, lines, out=None):
+        """rtx_psf_mtf: |DFT| of the two DEVICE lines (2, M), the first M//2
+        frequencies of each, into a DeviceArray (2, M//2).  Asynchronous."""
+        M = lines.shape[1]
+        if lines.shape != (2, M) or lines.dtype != np.float64:
+            raise ValueError("the lines must be a (2, M) float64 DeviceArray")
+        out = self.empty((2, M//2)) if out is None else out
+        check(self.lib.rtx_psf_mtf(self.ctx, M, lines.ptr, out.ptr))
+        return out
+
+    def psf_window(self, d_psf, i0, j0, w, out=None):
+        """rtx_psf_window: the (w, w) window of fftshift(psf) from shifted
+        index (i0, j0), indices modulo M, into a DeviceArray.  Asynchronous."""
+        M = self._square(d_psf)
+        out = self.empty((w, w)) if out is None else out
+        check(self.lib.rtx_psf_window(self.ctx, M, d_psf.ptr, int(i0), int(j0), int(w), out.ptr))
+        return out
+
+    def psf_metrics(self, d_psf, d, window=0):
+        """The figures Analysis.opds (rayopt/analysis.py:319-346) takes from a
+        PSF, computed on the DEVICE (M, M) FP64 PSF as rtx_psf writes it
+        (unshifted) whose frequency spacing is np.fft.fftfreq(M, d).  Only
+        O(M) bytes are transferred:
+
+        * x0, y0: the centroid (psf*x).sum(), (psf*y).sum() of the shifted
+          grids, from the line sums (math.fsum);
+        * dx: the node spacing; peak: psf.max();
+        * ee, r: the encircled energy cumsum(polar_sum(psf, (M/2 + x0/dx,
+          M/2 + y0/dx), "azimuthal")) and its radii arange(len(ee))*dx, summed
+          in 2^-62 fixed point (exact to M^2 2^-63);
+        * freq, mtf: fftfreq(M, dx)[:M//2] and (2, M//2) |DFT| of psf.sum(0)
+          and psf.sum(1), Analysis's order;
+        * window: None, or (x, y, psf) of the (2w+1)^2 nodes of the shifted
+          PSF around the centroid node, x and y relative to the centroid.
+
+        ValueError when an element is non-finite or outside [0, 2], the sum
+        exceeds 2 or w > (M-1)//2."""
+        M = self._square(d_psf)
+        w = int(window)
+        if w < 0 or w > (M - 1)//2:
+            raise ValueError("window %d is outside [0, %d] for M = %d" % (w, (M - 1)//2, M))
+        lines, peak, total, bad = self.psf_lines(d_psf)
+        try:
+            if bad or not total <= 2:
+                raise ValueError("the PSF has %d elements that are non-finite or outside [0, 2] "
+                                 "and sums to %r (at most 2 is needed)" % (bad, total))
+            cols, rows = lines.download()
+            f = np.fft.fftfreq(M, d)
+            x0, y0 = math.fsum(f*rows), math.fsum(f*cols)
+            fs = np.fft.fftshift(f)
+            dx = fs[1] - fs[0]
+            c0, c1 = M/2 + x0/dx, M/2 + y0/dx
+            corner = np.array([0., M - 1.])
+            rc = np.sqrt((corner[None, :] - c1)*(corner[None, :] - c1)
+                         + (corner[:, None] - c0)*(corner[:, None] - c0))
+            nbins = int(rc.max()) + 1
+            bins = self.psf_encircled(d_psf, c0, c1, nbins)
+            d_mtf = self.psf_mtf(lines)
+            try:
+                mtf = d_mtf.download()
+            finally:
+                d_mtf.free()
+        finally:
+            lines.free()
+        ee = np.cumsum(bins)/2.0**62
+        win = None
+        if w:
+            side = 2*w + 1
+            i0, j0 = math.floor(c0 + .5) - w, math.floor(c1 + .5) - w
+            d_win = self.psf_window(d_psf, i0, j0, side)
+            try:
+                pw = d_win.download()
+            finally:
+                d_win.free()
+            xw = fs[(i0 + np.arange(side)) % M] - x0
+            yw = fs[(j0 + np.arange(side)) % M] - y0
+            xw, yw = np.broadcast_arrays(xw[:, None], yw[None, :])
+            win = (xw, yw, pw)
+        return PsfMetrics(x0, y0, dx, peak, ee, np.arange(nbins)*dx,
+                          np.fft.fftfreq(M, dx)[:M//2], mtf, win)
 
     def ipc_export(self, darray):
         h = (C.c_ubyte*64)()

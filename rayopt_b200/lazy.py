@@ -508,6 +508,30 @@ class ResidentMixin:
         p, q = np.broadcast_arrays(f[:, None], f)
         return p, q, psf
 
+    def psf_metrics(self, pad=4, resample=4, regrid=None, window=0, **kw):
+        """The figures Analysis.opds (rayopt/analysis.py:319-346) takes from
+        psf() -- centroid, peak, encircled energy, MTF along both axes and
+        optionally a (2 window + 1)^2 window around the centroid -- computed
+        on the PSF in HBM (Engine.psf_metrics); the PSF itself never leaves
+        the device.  The OPD map comes from opd_map's `regrid`, as in
+        psf_device.  Returns an engine.PsfMetrics."""
+        radius = self.system[-1].distance                   # geometric_trace.py:147
+        m, _, x = self._opd_grid(radius, kw.pop("after", -2), kw.pop("image", -1), resample,
+                                 regrid)
+        if kw:
+            m.free()
+            raise TypeError("unexpected arguments %s" % sorted(kw))
+        eng = self._engine()
+        try:
+            d_psf = eng.psf(m, pad)
+        finally:
+            m.free()
+        try:
+            k = 1/(self.l/self.system.scale)                # :158-161
+            return eng.psf_metrics(d_psf, (x[1] - x[0])*k/radius, window)
+        finally:
+            d_psf.free()
+
 
 class ResidentTrace(ResidentMixin):
     """Standalone resident drop-in (no rayopt import needed) with launch rays
